@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the Lasso prover hot path on B200 (contract in the task prompt).
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload prove|msm] [--log-s 20]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic lookups:
     DensifiedRepresentation::from_lookup_indices -> commit -> SparsePolynomialEvaluationProof::prove
@@ -23,6 +24,10 @@ no data-path collective — proofs of different lookup batches are independent o
 --impl reference: the reference's own CPU implementation of the path = the oracle port (the Rust crate cannot
 be built in this image: no cargo/rustc, crates not vendored), all host threads, rank 0 only, the SAME 2^20 workload.
 --workload msm: BASELINE.json configs[4], the VariableBaseMSM-only sweep (tools/msm_bench.py holds the details).
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned to its caller (see
+dump_outputs); the inputs are seeded, so two builds run with the same arguments can be compared file by file.
+
+The benchmark writes nothing into the source tree (it may be read-only): no bytecode, no generator cache.
 """
 import argparse
 import hashlib
@@ -34,6 +39,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -50,6 +56,20 @@ make_inputs = wl.make_inputs
 def golden_cases():
     p = os.path.join(ROOT, "tests", "golden", "big_proofs.json")
     return json.load(open(p))["cases"] if os.path.exists(p) else {}
+
+
+def dump_outputs(d, commitment, proof, challenges):
+    """--dump-outputs: what commit + prove hand their caller, byte for byte, as float32 arrays (one value 0..255 per
+    byte): DIR/commitment.npy and DIR/proof.npy (the serialized bytes) and DIR/challenges.npy (one row of 32 bytes,
+    the four Montgomery limbs, per Fiat-Shamir challenge).  The library's output caps (4 MiB commitment, 4 MiB proof,
+    2^14 challenges) bound the three files to 34 MiB."""
+    os.makedirs(d, exist_ok=True)
+    chal = np.ascontiguousarray(challenges, dtype=np.uint64)
+    arrays = {"commitment": np.frombuffer(commitment, dtype=np.uint8),
+              "proof": np.frombuffer(proof, dtype=np.uint8),
+              "challenges": chal.view(np.uint8).reshape(chal.shape[0], 32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a.astype(np.float32))
 
 
 class ClockSampler:
@@ -142,7 +162,7 @@ def best_threads(C=4, log_m=16, log_probe=14):
     ncpu = os.cpu_count() or 8
     cands = sorted({t for t in (ncpu, ncpu // 2, ncpu // 4, 32, 16, 8) if 1 <= t <= ncpu}, reverse=True)
     idx, r, seed = make_inputs(log_probe, C, log_m, 4242)
-    gens = ol.generators(max((1 << ((log_probe + 3) - (log_probe + 3) // 2)) + 2, 600))
+    gens = ol.generators(max((1 << ((log_probe + 3) - (log_probe + 3) // 2)) + 2, 600), persist=False)
     best, best_t = None, None
     ol.lib().orc_set_num_threads(int(max(1, min(16, ncpu // 2))))
     ol.prove(KIND_XOR, C, log_m, 0, idx, r, gens, seed, flags=0)  # untimed: fault the heap in
@@ -162,7 +182,7 @@ def cpu_workload(log_s, C=4, log_m=16):
     import oracle_lib as ol
 
     idx, r, seed = make_inputs(log_s, C, log_m, wl.BENCH_SEED)
-    gens = np.ascontiguousarray(ol.generators(wl.gens_needed(C, log_s, C, log_m)))
+    gens = np.ascontiguousarray(ol.generators(wl.gens_needed(C, log_s, C, log_m), persist=False))
     return ol, idx, r, seed, gens
 
 
@@ -201,6 +221,8 @@ def run_reference(args):
         "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res["commitment"], res["proof"], res["challenges"])
     print(json.dumps(line))
 
 
@@ -265,7 +287,13 @@ def main():
     ap.add_argument("--no-batched", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true", help="N > 1: do not pin the host threads to the GPU's NUMA node")
     ap.add_argument("--no-sampler", action="store_true", help="diagnosis: no nvidia-smi clock sampler during the run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the commitment, proof and challenges of the last timed step to DIR/*.npy (prove workload)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload != "prove":
+        ap.error("--dump-outputs applies to the prove workload")
     if args.workload == "msm":
         run_msm(args)
         return
@@ -347,7 +375,7 @@ def main():
     ev0.record()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step_resident(dense)
+        last = step_resident(dense)
     ev1.record()
     barrier()
     wall = time.perf_counter() - t0
@@ -538,6 +566,8 @@ def main():
                                         "spans_ms": {k: round(v, 1) for k, v in res["spans"].items()}}
             except Exception as e:  # the checker failing must not hide the GPU number
                 line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": None, "kind": "port", "sample": "failed: %r" % e}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last[0], last[1].bytes, last[1].challenges)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

@@ -107,7 +107,9 @@ def f_op(which, op, a, b=None):
 _gens_cache = {}
 
 
-def generators(count, label=b"gens_sparse_poly"):
+def generators(count, label=b"gens_sparse_poly", persist=True):
+    """The first `count` points of the oracle's generator stream; persist=False never writes the on-disk cache (for
+    callers that must leave the source tree as they found it, such as bench.py)."""
     key = (label,)
     have = _gens_cache.get(key)
     if have is not None and have.shape[0] >= count:
@@ -118,7 +120,8 @@ def generators(count, label=b"gens_sparse_poly"):
     else:
         g = np.zeros((count, 8), dtype=np.uint64)
         lib().orc_sample_generators(sz(count), label, P(g))
-        np.save(cache, g)
+        if persist:
+            np.save(cache, g)
     _gens_cache[key] = g
     return g
 

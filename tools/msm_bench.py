@@ -41,7 +41,7 @@ def main(args):
         ctx.init_comm(rank, world)
     max_log = int(getattr(args, "msm_max_log", 24))
     cpu_max = 18
-    pool = np.ascontiguousarray(ol.generators(8194)[:8192])
+    pool = np.ascontiguousarray(ol.generators(8194, persist=False)[:8192])
     rows = []
     for log_n in range(16, max_log + 1, 2):
         n = 1 << log_n
