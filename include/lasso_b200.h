@@ -148,6 +148,22 @@ void lasso_gens_destroy(lasso_gens*);
 /* DensifiedRepresentation::from_lookup_indices  lasso/densified.rs:21-75.
  * indices: n_lookups x C row-major `usize` (the reference's &Vec<[usize; C]>). */
 int lasso_densify(lasso_ctx*, const uint64_t* indices, size_t n_lookups, size_t C, size_t log_m, lasso_dense** out);
+/* Element types of lasso_densify_device's index matrix. */
+enum { LASSO_IDX_U64 = 0, LASSO_IDX_I64 = 1, LASSO_IDX_U32 = 2, LASSO_IDX_I32 = 3 };
+/* DensifiedRepresentation::from_lookup_indices (lasso/densified.rs:21-75) on DEVICE-RESIDENT indices: the same result as
+ * lasso_densify, read in place from memory of the context's device (cudaMalloc'd or managed; e.g. a CUDA tensor).
+ * Element (k, d) of the n_lookups x C matrix is indices[k * row_stride + d * col_stride], strides in elements and >= 0
+ * (row-major: C, 1; column-major: 1, n_lookups; one column broadcast to all C dimensions: 1, 0), of type dtype
+ * (LASSO_IDX_*).  A negative index or one >= 2^log_m returns LASSO_ERR_INDEX_RANGE; bad shapes, strides or dtype
+ * LASSO_ERR_STRATEGY; a pointer that is not memory of the context's device < 0, before anything is allocated or
+ * launched.  The extent of the buffer is not checked: it must hold every element the strides address.
+ * Ordering: the call first waits (on the device) for the work already queued on cuda_stream (a cudaStream_t of the
+ * context's device; NULL = the legacy default stream), so a producer may still be writing the matrix when it is called.
+ * Lifetime: on return the library no longer reads the buffer; the caller may overwrite or free it at once.
+ * Sharded (after lasso_ctx_init_comm): collective, every rank passes a matrix with the same contents on its own device,
+ * and every rank reports the same result. */
+int lasso_densify_device(lasso_ctx*, const void* indices, int dtype, size_t n_lookups, size_t C, int64_t row_stride,
+                         int64_t col_stride, size_t log_m, void* cuda_stream, lasso_dense** out);
 void lasso_dense_destroy(lasso_dense*);
 size_t lasso_dense_s(const lasso_dense*);
 /* copies of the public fields (densified.rs:8-18) back to the host, for inspection / tests:

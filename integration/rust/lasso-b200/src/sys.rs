@@ -1,6 +1,6 @@
 //! Raw declarations of include/lasso_b200.h (one per C entry point; the header cites the reference item each replaces).
 #![allow(non_camel_case_types)]
-use std::os::raw::{c_char, c_int};
+use std::os::raw::{c_char, c_int, c_void};
 
 #[repr(C)]
 pub struct lasso_ctx {
@@ -58,6 +58,11 @@ extern "C" {
     pub fn lasso_gens_destroy(g: *mut lasso_gens);
     pub fn lasso_densify(ctx: *mut lasso_ctx, indices: *const u64, n_lookups: usize, c: usize, log_m: usize,
                          out: *mut *mut lasso_dense) -> c_int;
+    // indices: device memory of the context's device; dtype: LASSO_IDX_{U64 = 0, I64 = 1, U32 = 2, I32 = 3};
+    // cuda_stream: a cudaStream_t (null = legacy default stream)
+    pub fn lasso_densify_device(ctx: *mut lasso_ctx, indices: *const c_void, dtype: c_int, n_lookups: usize, c: usize,
+                                row_stride: i64, col_stride: i64, log_m: usize, cuda_stream: *mut c_void,
+                                out: *mut *mut lasso_dense) -> c_int;
     pub fn lasso_dense_destroy(d: *mut lasso_dense);
     pub fn lasso_dense_s(d: *const lasso_dense) -> usize;
     pub fn lasso_dense_read(ctx: *mut lasso_ctx, d: *const lasso_dense, which: c_int, out: *mut u64, cap_elems: usize) -> usize;

@@ -4,10 +4,12 @@ Field elements are numpy uint64 arrays (..., 4): ark-ff Montgomery limbs.  Affin
 extended points (..., 16)."""
 import ctypes as C
 import os
+import sys
 
 import numpy as np
 
 AND, OR, XOR, LT, RANGE_CHECK = 0, 1, 2, 3, 4
+IDX_U64, IDX_I64, IDX_U32, IDX_I32 = 0, 1, 2, 3  # LASSO_IDX_*: element types of lasso_densify_device
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -93,6 +95,7 @@ class Context:
         h = C.c_void_p()
         _chk(lib().lasso_ctx_create(C.byref(h), int(device)))
         self._h = h
+        self.device = int(device)
         self._scratch = {}
 
     def _buf(self, name, shape, dtype):
@@ -315,6 +318,11 @@ class SparsePolyCommitmentGens:
             pass
 
 
+def _is_cuda_tensor(x):
+    torch = sys.modules.get("torch")  # a tensor implies torch is loaded; api.py never imports it itself
+    return torch is not None and isinstance(x, torch.Tensor) and x.is_cuda
+
+
 class DensifiedRepresentation:
     """src/lasso/densified.rs:8-96 (device resident)"""
 
@@ -325,12 +333,38 @@ class DensifiedRepresentation:
 
     @classmethod
     def from_lookup_indices(cls, ctx, indices, log_m):
+        """indices: n x C lookup indices.  A CUDA torch.Tensor (int64, uint64, int32 or uint32, any strides) on the
+        context's device is read in place, after the work queued on the current stream of its device; anything else is
+        converted to a host uint64 array."""
+        if _is_cuda_tensor(indices):
+            return cls._from_cuda_tensor(ctx, indices, log_m)
         idx = np.ascontiguousarray(indices, dtype=np.uint64)
         assert idx.ndim == 2
         h = C.c_void_p()
         _chk(lib().lasso_densify(ctx._h, _p(idx), C.c_size_t(idx.shape[0]), C.c_size_t(idx.shape[1]),
                                  C.c_size_t(log_m), C.byref(h)))
         return cls(ctx, h, idx.shape[1], log_m)
+
+    @classmethod
+    def _from_cuda_tensor(cls, ctx, t, log_m):
+        import torch
+
+        codes = {torch.int64: IDX_I64, torch.int32: IDX_I32}
+        for name, code in (("uint64", IDX_U64), ("uint32", IDX_U32)):
+            if hasattr(torch, name):
+                codes[getattr(torch, name)] = code
+        if t.dim() != 2:
+            raise TypeError("lookup indices must be a 2-D (n, C) tensor, got shape %s" % (tuple(t.shape),))
+        if t.dtype not in codes:
+            raise TypeError("lookup indices must be int64, uint64, int32 or uint32, got %s" % t.dtype)
+        if t.device.index != ctx.device:
+            raise ValueError("lookup indices are on cuda:%d, the context on cuda:%d" % (t.device.index, ctx.device))
+        stream = torch.cuda.current_stream(t.device).cuda_stream
+        h = C.c_void_p()
+        _chk(lib().lasso_densify_device(ctx._h, C.c_void_p(t.data_ptr()), codes[t.dtype], C.c_size_t(t.shape[0]),
+                                        C.c_size_t(t.shape[1]), C.c_int64(t.stride(0)), C.c_int64(t.stride(1)),
+                                        C.c_size_t(log_m), C.c_void_p(stream), C.byref(h)))
+        return cls(ctx, h, t.shape[1], log_m)
 
     def _read(self, which, n, width):
         out = np.zeros((n, width) if width > 1 else (n,), dtype=np.uint64)

@@ -460,6 +460,22 @@ int lasso_densify(lasso_ctx* h, const uint64_t* indices, size_t n_lookups, size_
   return 0;
   LB_CATCH
 }
+int lasso_densify_device(lasso_ctx* h, const void* indices, int dtype, size_t n_lookups, size_t C, int64_t row_stride,
+                         int64_t col_stride, size_t log_m, void* cuda_stream, lasso_dense** out) {
+  LB_TRY_CTX(h)
+  *out = nullptr;
+  auto t0 = std::chrono::steady_clock::now();
+  int err = 0;
+  Dense* d = densify_device(h->c, indices, dtype, n_lookups, C, row_stride, col_stride, log_m,
+                            static_cast<cudaStream_t>(cuda_stream), &err);
+  if (!d)
+    return err == 3 ? fail(LASSO_ERR_INDEX_RANGE, "densify_device: lookup index negative or >= m")
+                    : fail(LASSO_ERR_STRATEGY, "densify_device: invalid shape, strides or index type");
+  h->c->t_densify_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  *out = new lasso_dense{d};
+  return 0;
+  LB_CATCH
+}
 void lasso_dense_destroy(lasso_dense* d) {
   if (!d) return;
   delete d->d;

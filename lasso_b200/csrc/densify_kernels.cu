@@ -6,8 +6,8 @@
 // index k) then has read[k] = p - start[a], start = the exclusive scan of the per-address counts (= final).
 // The stable sort is an LSD radix sort with 8-bit digits over packed (address << 32 | k) words, all C dimensions
 // in the same launches (blockIdx.y = dimension):
-//   extract_kernel   column `dim` of the row-major index matrix -> packed words (zero-padded to s, densified.rs:33-37),
-//                    this rank's shard of dim, per-address counts (RED atomics)
+//   extract_kernel   column `dim` of the strided index matrix -> packed words (zero-padded to s, densified.rs:33-37),
+//                    range check (densified.rs:46), this rank's shard of dim, per-address counts (RED atomics)
 //   per 8-bit digit (ceil(log_m / 8) passes):
 //     radix_hist_kernel     digit histogram of every tile of 2048 elements -> H[dim][bin][tile]
 //     scan_*_kernel         exclusive scan of H in (bin, tile) order = where each tile's run of each digit starts
@@ -18,6 +18,8 @@
 // Integer, order-preserving, bit-identical to the sequential scan for every input (skew included: nothing here depends
 // on how the addresses are distributed).  A few launches of ~10-40 us for 2^20 accesses x 4 dimensions where the host
 // scan needs ~3 ms on C threads; no 2^log_m table in shared memory, so any log_m <= 31.
+#include <type_traits>
+
 #include "kernels.cuh"
 
 namespace lb {
@@ -28,16 +30,31 @@ static constexpr int kRadixTile = kRadixThreads * kRadixRounds;  // 2048 element
 static constexpr uint32_t kDzScanTile = 4096;
 
 // ---------------------------------------------------------------------------------------------- extract
-// idx: n x C u32 row-major (already narrowed and range-checked on the host while staging it into pinned memory)
+// Element (k, dim) of the n x C index matrix is idx[k * row_stride + dim * col_stride] (element strides >= 0: row-major,
+// column-major and broadcast layouts are read in place).  An index that is negative or >= m (densified.rs:46) raises
+// *bad (when bad is non-null) and is counted as address 0, so the count atomics below never leave the m counters.
+// The host-staged path passes u32 (narrowed and range-checked on the host while staging) with no flag.
+template <class T>
+__device__ __forceinline__ bool dz_in_range(T v, uint32_t m) {
+  if constexpr (std::is_signed<T>::value) return v >= 0 && (uint64_t)v < m;
+  else return (uint64_t)v < m;
+}
+template <class T>
 __global__ void __launch_bounds__(256)
-    dz_extract_kernel(const uint32_t* idx, size_t n, size_t s, int C, uint32_t m, int G, int g, unsigned long long* packed,
-                      uint32_t* count, uint32_t* dim_loc_base, size_t dim_stride) {
+    dz_extract_kernel(const T* idx, int64_t row_stride, int64_t col_stride, size_t n, size_t s, uint32_t m, int G, int g,
+                      unsigned long long* packed, uint32_t* count, uint32_t* dim_loc_base, size_t dim_stride, uint32_t* bad) {
   const int dim = blockIdx.y;
+  const T* col = idx + (int64_t)dim * col_stride;
   unsigned long long* out = packed + (size_t)dim * s;
   uint32_t* cnt = count + (size_t)dim * m;
   uint32_t* dim_loc = dim_loc_base + (size_t)dim * dim_stride;
   for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < s; k += (size_t)gridDim.x * blockDim.x) {
-    const uint32_t a = k < n ? idx[k * C + dim] : 0u;
+    uint32_t a = 0u;
+    if (k < n) {
+      const T v = col[(int64_t)k * row_stride];
+      if (dz_in_range(v, m)) a = (uint32_t)v;
+      else if (bad) *bad = 1u;
+    }
     out[k] = ((unsigned long long)a << 32) | (unsigned long long)k;
     atomicAdd(cnt + a, 1u);
     if ((int)(k % G) == g) dim_loc[k / G] = a;
@@ -221,9 +238,9 @@ size_t densify_scratch_words(size_t s, int C, size_t log_m) {
   const size_t tsums = (size_t)C * ((scan_len + kDzScanTile - 1) / kDzScanTile + 1);
   return 2 * 2 * (size_t)C * s /* two packed arrays of u64 */ + (size_t)C * m /* counts / start */ + H + tsums + 64;
 }
-// d_idx: n x C u32 on the device.  Outputs are this rank's shards: dim_i at dim_loc + i * dim_stride (likewise
+// src: the n x C index matrix on the device.  Outputs are this rank's shards: dim_i at dim_loc + i * dim_stride (likewise
 // read, final).  Returns the number of kernels launched.
-int launch_densify(const uint32_t* d_idx, size_t n, size_t s, int C, size_t log_m, int G, int g, uint32_t* scratch,
+int launch_densify(const DzSource& src, size_t n, size_t s, int C, size_t log_m, int G, int g, uint32_t* scratch,
                    uint32_t* dim_loc, size_t dim_stride, uint32_t* read_loc, size_t read_stride, uint32_t* final_loc,
                    size_t final_stride, cudaStream_t st) {
   const uint32_t m = 1u << log_m;
@@ -238,9 +255,24 @@ int launch_densify(const uint32_t* d_idx, size_t n, size_t s, int C, size_t log_
   {
     size_t bx = (s + 255) / 256;
     if (bx > (size_t)kNumSMs * 8) bx = kNumSMs * 8;
-    dz_extract_kernel<<<dim3((unsigned)bx, (unsigned)C), 256, 0, st>>>(d_idx, n, s, C, m, G, g, pa, count, dim_loc, dim_stride);
+    const dim3 grid((unsigned)bx, (unsigned)C);
+#define LB_DZ_EXTRACT(T)                                                                                                \
+  dz_extract_kernel<T><<<grid, 256, 0, st>>>(static_cast<const T*>(src.p), src.row_stride, src.col_stride, n, s, m, G, g, \
+                                             pa, count, dim_loc, dim_stride, src.bad)
+    switch (src.type) {
+      case kDzU64: LB_DZ_EXTRACT(uint64_t); break;
+      case kDzI64: LB_DZ_EXTRACT(int64_t); break;
+      case kDzU32: LB_DZ_EXTRACT(uint32_t); break;
+      case kDzI32: LB_DZ_EXTRACT(int32_t); break;
+      default: throw std::runtime_error("launch_densify: unknown index type");
+    }
+#undef LB_DZ_EXTRACT
     LB_LAUNCH_CHECK();
     launches++;
+    if (src.bad_host) {  // the verdict travels to the host while the sort below is already queued
+      LB_CUDA_CHECK(cudaMemcpyAsync(src.bad_host, src.bad, 4, cudaMemcpyDeviceToHost, st));
+      LB_CUDA_CHECK(cudaEventRecord(src.bad_ready, st));
+    }
   }
   unsigned long long *cur = pa, *nxt = pb;
   for (int shift = 0; shift < (int)log_m; shift += 8) {  // LSD: least significant digit first, every pass stable

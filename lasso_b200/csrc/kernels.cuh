@@ -149,9 +149,22 @@ void launch_scale(const fr_t* in, fr_t* out, size_t n, const fr_t& k, cudaStream
 void densify_init_device();
 bool densify_gpu_supported(size_t s, size_t log_m);
 size_t densify_scratch_words(size_t s, int C, size_t log_m);
-// d_idx: n x C u32 (device).  All C dimensions at once; outputs are this rank's shards (rank g of G: accesses k = i*G + g,
-// addresses a = i*G + g): dim_i at dim_loc + i*dim_stride, read_i at read_loc + i*read_stride, final_i likewise.
-int launch_densify(const uint32_t* d_idx, size_t n, size_t s, int C, size_t log_m, int G, int g, uint32_t* scratch,
+// The n x C index matrix on the device: element (k, dim) at p + k*row_stride + dim*col_stride (elements, >= 0), of one of
+// four integer types (the values of LASSO_IDX_*).  bad (may be null): raised by the extract when an index is negative or
+// >= m (that index is then counted as address 0).  bad_host (may be null, needs bad): pinned word the flag is copied
+// to right after the extract, followed by a record of bad_ready, so the host can wait for the verdict alone.
+enum { kDzU64 = 0, kDzI64 = 1, kDzU32 = 2, kDzI32 = 3 };
+struct DzSource {
+  const void* p = nullptr;
+  int type = kDzU32;
+  int64_t row_stride = 0, col_stride = 1;
+  uint32_t* bad = nullptr;
+  uint32_t* bad_host = nullptr;
+  cudaEvent_t bad_ready = nullptr;
+};
+// All C dimensions at once; outputs are this rank's shards (rank g of G: accesses k = i*G + g, addresses a = i*G + g):
+// dim_i at dim_loc + i*dim_stride, read_i at read_loc + i*read_stride, final_i likewise.
+int launch_densify(const DzSource& src, size_t n, size_t s, int C, size_t log_m, int G, int g, uint32_t* scratch,
                    uint32_t* dim_loc, size_t dim_stride, uint32_t* read_loc, size_t read_stride, uint32_t* final_loc,
                    size_t final_stride, cudaStream_t st);
 

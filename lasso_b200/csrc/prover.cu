@@ -240,6 +240,7 @@ Ctx* ctx_create(int device) {
   densify_init_device();
   LB_CUDA_CHECK(cudaEventCreateWithFlags(&c->ev_aux, cudaEventDisableTiming));
   LB_CUDA_CHECK(cudaEventCreateWithFlags(&c->ev_stage, cudaEventDisableTiming));
+  LB_CUDA_CHECK(cudaEventCreateWithFlags(&c->ev_input, cudaEventDisableTiming));
   const char* sp = getenv("LASSO_B200_SPANS");
   c->span_sync = sp && sp[0] == '1';
   return c.release();
@@ -254,6 +255,7 @@ void ctx_destroy(Ctx* c) {
   cudaFree(c->d_flag);
   if (c->ev_aux) cudaEventDestroy(c->ev_aux);
   if (c->ev_stage) cudaEventDestroy(c->ev_stage);
+  if (c->ev_input) cudaEventDestroy(c->ev_input);
   if (c->h_stage) cudaFreeHost(c->h_stage);
   if (c->h_mapped) cudaFreeHost(c->h_mapped);
   if (c->h_pub && c->h_pub_owned) cudaFreeHost(c->h_pub);
@@ -493,14 +495,14 @@ static std::vector<uint8_t> commit_u32(Ctx* c, const Gens& g, const uint32_t* d_
 }
 
 // ---------------------------------------------------------------------------------------------- densify
-Dense* densify(Ctx* c, const uint64_t* indices, size_t n, size_t C, size_t log_m, int* err) {
-  SpanTimer sp(c, "Densify");
+// The shape checks both densify entry points share and the header of their result (nullptr with *err = 4 if invalid).
+static std::unique_ptr<Dense> dense_header(Ctx* c, size_t n, size_t C, size_t log_m, int* err) {
   *err = 0;
   if (n == 0 || C == 0 || C > 16 || log_m < 1 || log_m > 28) {
     *err = 4;
     return nullptr;
   }
-  const size_t G = (size_t)c->world, gr = (size_t)c->rank;
+  const size_t G = (size_t)c->world;
   std::unique_ptr<Dense> d(new Dense());
   d->ctx = c;
   d->C = C;
@@ -509,14 +511,41 @@ Dense* densify(Ctx* c, const uint64_t* indices, size_t n, size_t C, size_t log_m
   d->m = (size_t)1 << log_m;
   d->nv_l = log2_exact_or_ceil(next_pow2(2 * C * d->s));
   d->nv_m = log2_exact_or_ceil(next_pow2(C)) + log_m;
-  const size_t s = d->s, m = d->m;
-  if (G > 1 && (s < 2 * G || m < 2 * G)) {
+  if (G > 1 && (d->s < 2 * G || d->m < 2 * G)) {
     *err = 4;
     return nullptr;
   }
-  d->s_loc = s / G;
-  d->m_loc = m / G;
-  const size_t s_loc = d->s_loc, m_loc = d->m_loc;
+  d->s_loc = d->s / G;
+  d->m_loc = d->m / G;
+  return d;
+}
+
+// The device half both entry points share once the index matrix is on the device: the four arrays of d and their zero
+// padding, the stable sort by address (densify_kernels.cu) and DensePolynomial::from_usize + merge.  Queued on the
+// context stream, no sync.
+static void densify_on_device(Ctx* c, Dense* d, const DzSource& src, size_t n) {
+  const size_t G = (size_t)c->world, gr = (size_t)c->rank, C = d->C, s = d->s, s_loc = d->s_loc, m_loc = d->m_loc;
+  const size_t nl = ((size_t)1 << d->nv_l) / G, nm = ((size_t)1 << d->nv_m) / G;  // local lengths
+  d->d_l_u32.alloc(c, nl);
+  d->d_m_u32.alloc(c, nm);
+  d->d_l_fr.alloc(c, nl);
+  d->d_m_fr.alloc(c, nm);
+  DBuf<uint32_t> scratch(c, densify_scratch_words(s, (int)C, d->log_m));
+  if (nl > 2 * C * s_loc) LB_CUDA_CHECK(cudaMemsetAsync(d->d_l_u32.p + 2 * C * s_loc, 0, (nl - 2 * C * s_loc) * 4, c->st));
+  if (nm > C * m_loc) LB_CUDA_CHECK(cudaMemsetAsync(d->d_m_u32.p + C * m_loc, 0, (nm - C * m_loc) * 4, c->st));
+  g_launches += launch_densify(src, n, s, (int)C, d->log_m, (int)G, (int)gr, scratch.p, d->d_l_u32.p, s_loc,
+                               d->d_l_u32.p + C * s_loc, s_loc, d->d_m_u32.p, m_loc, c->st);
+  launch_from_u32(d->d_l_u32.p, d->d_l_fr.p, nl, c->st);  // DensePolynomial::from_usize + merge
+  launch_from_u32(d->d_m_u32.p, d->d_m_fr.p, nm, c->st);
+  g_launches += 2;
+}
+
+Dense* densify(Ctx* c, const uint64_t* indices, size_t n, size_t C, size_t log_m, int* err) {
+  SpanTimer sp(c, "Densify");
+  std::unique_ptr<Dense> d = dense_header(c, n, C, log_m, err);
+  if (!d) return nullptr;
+  const size_t G = (size_t)c->world, gr = (size_t)c->rank;
+  const size_t s = d->s, m = d->m, s_loc = d->s_loc, m_loc = d->m_loc;
   const size_t nl = ((size_t)1 << d->nv_l) / G, nm = ((size_t)1 << d->nv_m) / G;  // local lengths
   {
     const char* hd = getenv("LASSO_B200_HOST_DENSIFY");
@@ -529,10 +558,6 @@ Dense* densify(Ctx* c, const uint64_t* indices, size_t n, size_t C, size_t log_m
     if (densify_gpu_supported(s, log_m) && want_gpu && !(hd && hd[0] == '1')) {
       // upload the raw index matrix, derive dim / read / final on the device.  When one proof is sharded every rank
       // does this for the whole sequence and stores only its shard.
-      d->d_l_u32.alloc(c, nl);
-      d->d_m_u32.alloc(c, nm);
-      d->d_l_fr.alloc(c, nl);
-      d->d_m_fr.alloc(c, nm);
       // narrow usize -> u32 (and range-check, densified.rs:46) while staging into pinned memory: half the PCIe
       // bytes and a full-rate copy.  Pipelined: the matrix is cut into pieces, a few host threads narrow them
       // round-robin, and the upload of a piece starts as soon as it is staged (the copy of the early pieces overlaps
@@ -550,7 +575,6 @@ Dense* densify(Ctx* c, const uint64_t* indices, size_t n, size_t C, size_t log_m
       const uint64_t* src = indices + row0 * C;
       uint32_t* stage = c->stage(std::max<size_t>(total, 1));
       DBuf<uint32_t> d_idx(c, G * rows_per * C), d_mine(c, G > 1 ? rows_per * C : 0);
-      DBuf<uint32_t> scratch(c, densify_scratch_words(s, (int)C, log_m));
       uint32_t* d_dst = G > 1 ? d_mine.p : d_idx.p;
       {
         const size_t npieces = total >= (1u << 20) ? 64 : 1, nthreads = npieces > 1 ? (total >= (1u << 25) ? 16 : total >= (1u << 22) ? 8 : 4) : 1;
@@ -610,13 +634,12 @@ Dense* densify(Ctx* c, const uint64_t* indices, size_t n, size_t C, size_t log_m
         }
         if (G > 1) comm_allgather(c, d_mine.p, d_idx.p, rows_per * C * sizeof(uint32_t));
       }
-      if (nl > 2 * C * s_loc) LB_CUDA_CHECK(cudaMemsetAsync(d->d_l_u32.p + 2 * C * s_loc, 0, (nl - 2 * C * s_loc) * 4, c->st));
-      if (nm > C * m_loc) LB_CUDA_CHECK(cudaMemsetAsync(d->d_m_u32.p + C * m_loc, 0, (nm - C * m_loc) * 4, c->st));
-      g_launches += launch_densify(d_idx.p, n, s, (int)C, log_m, (int)G, (int)gr, scratch.p, d->d_l_u32.p, s_loc,
-                                   d->d_l_u32.p + C * s_loc, s_loc, d->d_m_u32.p, m_loc, c->st);
-      launch_from_u32(d->d_l_u32.p, d->d_l_fr.p, nl, c->st);  // DensePolynomial::from_usize + merge
-      launch_from_u32(d->d_m_u32.p, d->d_m_fr.p, nm, c->st);
-      g_launches += 2;
+      DzSource staged;  // n x C u32 row-major, range-checked above
+      staged.p = d_idx.p;
+      staged.type = kDzU32;
+      staged.row_stride = (int64_t)C;
+      staged.col_stride = 1;
+      densify_on_device(c, d.get(), staged, n);
       // no stream sync here: everything downstream is stream-ordered, and the staging buffer is guarded by ev_stage
       return d.release();
     }
@@ -686,6 +709,50 @@ Dense* densify(Ctx* c, const uint64_t* indices, size_t n, size_t C, size_t log_m
   launch_from_u32(d->d_m_u32.p, d->d_m_fr.p, nm, c->st);
   g_launches += 2;
   c->sync();
+  return d.release();
+}
+
+// densified.rs:21-75 on an index matrix the caller already holds on the context's device (any of four integer types,
+// element strides >= 0).  Ordered after the work queued on `producer`; returns once the extract has read the matrix
+// and the range verdict is on the host (the sort and the field conversion stay queued).  Sharded: collective, every
+// rank passes the same matrix on its own device, extracts its shard and checks every element itself.
+Dense* densify_device(Ctx* c, const void* d_idx, int dtype, size_t n, size_t C, int64_t row_stride, int64_t col_stride,
+                      size_t log_m, cudaStream_t producer, int* err) {
+  SpanTimer sp(c, "Densify");
+  std::unique_ptr<Dense> d = dense_header(c, n, C, log_m, err);
+  if (!d) return nullptr;
+  if (!densify_gpu_supported(d->s, log_m) || row_stride < 0 || col_stride < 0 || dtype < kDzU64 || dtype > kDzI32) {
+    *err = 4;
+    return nullptr;
+  }
+  cudaPointerAttributes pa;
+  if (cudaPointerGetAttributes(&pa, d_idx) != cudaSuccess) {
+    cudaGetLastError();  // an unknown pointer: clear the (non-sticky) error it left behind
+    pa.type = cudaMemoryTypeUnregistered;
+  }
+  if (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged)
+    throw std::invalid_argument("densify_device: the indices are not device memory (host buffers go to lasso_densify)");
+  if (pa.device != c->device)
+    throw std::invalid_argument("densify_device: the indices are memory of device " + std::to_string(pa.device) +
+                                ", the context is on device " + std::to_string(c->device));
+  LB_CUDA_CHECK(cudaEventRecord(c->ev_input, producer));
+  LB_CUDA_CHECK(cudaStreamWaitEvent(c->st, c->ev_input, 0));
+  DBuf<uint32_t> bad(c, 1);
+  LB_CUDA_CHECK(cudaMemsetAsync(bad.p, 0, 4, c->st));
+  DzSource src;
+  src.p = d_idx;
+  src.type = dtype;
+  src.row_stride = row_stride;
+  src.col_stride = col_stride;
+  src.bad = bad.p;
+  src.bad_host = reinterpret_cast<uint32_t*>(c->h_pin);
+  src.bad_ready = c->ev_aux;
+  densify_on_device(c, d.get(), src, n);
+  LB_CUDA_CHECK(cudaEventSynchronize(c->ev_aux));  // the extract is done: the caller's matrix is no longer read
+  if (*src.bad_host) {
+    *err = 3;
+    return nullptr;  // d's arrays go back to the pool in stream order, behind the queued sort
+  }
   return d.release();
 }
 

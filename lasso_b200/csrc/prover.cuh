@@ -68,6 +68,7 @@ struct Ctx {
   cudaEvent_t ev_aux = nullptr;  // marks a device->host copy that overlaps later launches on the same stream
   cudaEvent_t ev_stage = nullptr;  // recorded after the last upload out of h_stage (the buffer is reused by the next densify)
   bool stage_busy = false;
+  cudaEvent_t ev_input = nullptr;  // recorded on the caller's stream: densify_device waits there for its input's producer
   // host-thread placement (bind_host_threads): the CPUs the library's helper threads may use
   cpu_set_t helper_mask;
   bool have_helper_mask = false;
@@ -277,6 +278,9 @@ Gens* gens_create(Ctx*, const uint64_t* stream_affine, size_t n_points, size_t c
                   size_t log_m);
 size_t gens_points_needed(size_t c, size_t s, size_t num_memories, size_t log_m);
 Dense* densify(Ctx*, const uint64_t* indices, size_t n_lookups, size_t C, size_t log_m, int* err);
+// the same on an n x C matrix already on the context's device (dtype: kDzU64 .. kDzI32, element strides)
+Dense* densify_device(Ctx*, const void* d_idx, int dtype, size_t n_lookups, size_t C, int64_t row_stride, int64_t col_stride,
+                      size_t log_m, cudaStream_t producer, int* err);
 std::vector<uint8_t> commit(Ctx*, const Dense&, const Gens&);
 std::vector<uint8_t> prove(Ctx*, const Strategy& S, Dense&, const std::vector<fr_t>& r, const Gens&,
                            const std::string& transcript_label, const std::string& tape_label, const fr_t& tape_seed,
